@@ -305,6 +305,8 @@ def main() -> None:
     ap.add_argument("--resident-only", action="store_true", help="only the device-resident measurement (no e2e loops)")
     ap.add_argument("--profile-bf16", action="store_true",
                     help="profiling aid: run ONLY plain-bf16 forwards and print nothing (for ncu captures)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step (fp32, inputs resident) returned as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "mscnn_b200" else args.warmup
     if args.impl == "reference":
@@ -461,7 +463,22 @@ def main() -> None:
             step_resident()
         torch.cuda.synchronize()
         return
+
+    def outputs() -> dict:
+        """What a caller of the timed path receives: the net's outputs and the final detections (or, with the
+        exchange on, the gathered payload of every rank), as float32 / float64 arrays."""
+        out = {name: net.blob(name).astype(np.float32) for name in net.outputs}
+        if use_peer:
+            out["gathered_payload"] = xchg.gathered().cpu().numpy().astype(np.float32)
+        elif use_gather:
+            out["gathered_payload"] = payload_all.cpu().numpy().astype(np.float32)
+        else:
+            out["detections"] = dets.cpu().numpy().astype(np.float32)
+            out["detection_counts"] = cnt.cpu().numpy().astype(np.float64)
+        return out
+
     results = {}
+    dumped = None
     sampler = ClockSampler(local)      # every rank samples ITS GPU: the scaling analysis needs the slowest one's clocks
     for mode in (["fp32"] if args.no_bf16 else ["fp32", "bf16"]):
         mnet.set_precision(mode)
@@ -469,6 +486,8 @@ def main() -> None:
             sampler.start()
         ms = timed(step_resident, args.steps, args.warmup)
         launched = timed.launched
+        if mode == "fp32" and args.dump_outputs and rank == 0:
+            dumped = outputs()
         step_ms = sorted(timed.step_ms)
         clocks = sampler.stop() if (mode == "fp32" and sampler) else None
         per_rank = None
@@ -522,6 +541,11 @@ def main() -> None:
         if world > 1:
             dist.destroy_process_group()
         return
+    if dumped is not None:
+        d = Path(args.dump_outputs)
+        d.mkdir(parents=True, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(d / f"{name}.npy", a)
     pk = peaks()
 
     def roofline(r, pk):

@@ -50,6 +50,14 @@ def available() -> bool:
     return LIB.exists()
 
 
+def present(p: Path) -> bool:
+    """exists() that treats a reference tree this user may not read as absent (exists() raises on EACCES)."""
+    try:
+        return p.exists()
+    except OSError:
+        return False
+
+
 KITTI_EVAL_SRC = REF / "examples" / "kitti_result" / "eval" / "evaluate_object.cpp"
 KITTI_EVAL_BIN = OUT / "evaluate_object"
 
@@ -57,7 +65,7 @@ KITTI_EVAL_BIN = OUT / "evaluate_object"
 def build_kitti_eval(force: bool = False) -> Path | None:
     """The reference's KITTI evaluation tool (examples/kitti_result/eval/evaluate_object.cpp), a stand-alone
     program with no dependency beyond libstdc++: compiled verbatim from where it lies."""
-    if not KITTI_EVAL_SRC.exists():
+    if not present(KITTI_EVAL_SRC):
         return KITTI_EVAL_BIN if KITTI_EVAL_BIN.exists() else None
     if KITTI_EVAL_BIN.exists() and not force and KITTI_EVAL_SRC.stat().st_mtime <= KITTI_EVAL_BIN.stat().st_mtime:
         return KITTI_EVAL_BIN
@@ -70,7 +78,7 @@ def build_kitti_eval(force: bool = False) -> Path | None:
 
 def build(force: bool = False) -> Path | None:
     build_kitti_eval(force)
-    if not REF.exists():
+    if not present(REF):
         return LIB if LIB.exists() else None
     srcs = [REF / s for s in REF_SOURCES] + OWN_SOURCES
     deps = srcs + list(SHIM.rglob("*.h*")) + list((ROOT / "mscnn_b200/csrc/proto_shared").rglob("*.h*")) + [Path(__file__)]

@@ -20,6 +20,14 @@ Outputs (committed):
                        head outputs (`python tests/golden/make_golden.py full`).
   e2e_wider_768x1024.npz  WIDER FACE mscnn-12s-2x at 1x3x768x1024 (configs[4]).
   e2e_7s2x_576x1920.npz   mscnn-7s-576-2x at 1x3x576x1920 (configs[1]).
+  port_vs_reference.npz   the reference's output blobs for the seeded single-layer cases of tests/test_oracle.py
+                       (`python tests/golden/make_golden.py port`).
+  isolated_*.npz       the detection stages of mscnn-7s (1x3x96x320) and of both cascade nets fed with the reference's
+                       own proposals and a seeded feature map (tests/test_net_gpu.py _synthetic_map): the proposals, the
+                       map's scale and the stage outputs (every 16th row of the WIDER cascade; roi_c1 / fc6
+                       sub-sampled) (`python tests/golden/make_golden.py isolated`).
+  shipped_deploy_nets.json  sha256 digests of the structure of six of the reference's shipped deploy files as this
+                       parser loads them (`python tests/golden/make_golden.py deploy`).
 """
 import sys
 from pathlib import Path
@@ -32,6 +40,7 @@ from mscnn_b200 import models, synth
 from oracle import ref
 
 OUT = Path(__file__).resolve().parent
+sys.path.insert(0, str(OUT.parent))
 SUB = 7919  # subsample stride (prime)
 
 
@@ -221,6 +230,79 @@ def main_full(which=("8s", "wider", "7s2x")):
         print("e2e_7s2x_576x1920: proposals", g["proposals"].shape, f"{time.time() - t:.0f} s", flush=True)
 
 
+PORT_ALIGN_ROW_STEP = 6
+
+
+def main_port():
+    import test_oracle
+    vec = {}
+    for case, make in test_oracle.PORT_CASES.items():
+        proto, params, blobs, outputs = make()
+        net = ref.RefNet(proto, is_path=False)
+        for layer, arrs in params.items():
+            for k, a in enumerate(arrs):
+                net.set_param(layer, k, a)
+        for name, a in blobs.items():
+            net.set_blob(name, a)
+        net.forward()
+        vec.update({f"{case}__{o}": net.blob(o) for o in outputs})
+    vec["cascade_layers__a"] = vec["cascade_layers__a"][::PORT_ALIGN_ROW_STEP].copy()     # a fixed sample of the ROIs
+    np.savez_compressed(OUT / "port_vs_reference.npz", **vec)
+    print("port_vs_reference.npz:", {k: v.shape for k, v in vec.items()})
+
+
+SUB_ISOLATED = 997
+ROW_STEP = {"cascade_kitti": 1, "cascade_wider": 16}
+CASCADE_STAGES = ["cls_pred", "bbox_pred", "proposals_2nd", "cls_pred_2nd", "bbox_pred_2nd", "proposals_3rd", "cls_pred_3rd",
+                  "bbox_pred_3rd", "output_bbox_1st", "output_bbox_2nd", "output_bbox_3rd", "cls_prob_1st", "cls_prob_2nd",
+                  "cls_prob_3rd"]
+
+
+def main_isolated():
+    """Each net runs once end to end for its proposals; then its feature map is replaced by the seeded stand-in (same
+    shape, same second moment) and the stages after it run again."""
+    from test_net_gpu import _isolated_protos, _synthetic_map
+    for kind, (proto, (n, h, w), feat, first) in _isolated_protos().items():
+        net = ref.RefNet(proto, is_path=False)
+        layers = [(nm, t, net.param_shapes(nm)) for nm, t in zip(net.layer_names, net.layer_types)]
+        net.set_params(synth.make_weights(layers))
+        net.set_blob("data", synth.make_images(n, h, w))
+        net.forward()
+        real = net.blob(feat)
+        scale = np.float64(np.sqrt(np.mean(real.astype(np.float64) ** 2) * 2))   # E[relu(z)^2] = 1/2
+        fmap = _synthetic_map(real.shape, scale)
+        net.set_blob(feat, fmap)             # the harness inserts no Split layers: every reader reads this blob
+        net.forward(first)
+        g = {"proposals": net.blob("proposals"), "fmap_scale": np.array([scale])}
+        if kind == "head_7s":
+            for b in ("cls_pred", "bbox_pred"):
+                g[b] = net.blob(b)
+            for b in ("roi_c1", "fc6"):
+                x = net.blob(b)
+                g[b + "__sub"] = x.reshape(-1)[::SUB_ISOLATED].copy()
+                g[b + "__m2"] = np.array([np.mean(x.astype(np.float64) ** 2)])
+                g[b + "__shape"] = np.array(x.shape, dtype=np.int64)
+        else:
+            # every row runs through the stages on its own: a fixed sample of the rows is stored
+            g["rows"] = np.arange(0, len(g["proposals"]), ROW_STEP[kind])
+            for b in CASCADE_STAGES + (["cls_prob_1st_3rd", "cls_prob_2nd_3rd", "cls_prob_3rd_avg"] if kind == "cascade_wider" else []):
+                x = net.blob(b)
+                g[b] = x[g["rows"]]
+                g[b + "__shape"] = np.array(x.shape, dtype=np.int64)
+        np.savez_compressed(OUT / f"isolated_{kind}.npz", **g)
+        print(f"isolated_{kind}: proposals", g["proposals"].shape)
+
+
+def main_deploy():
+    """shipped_deploy_nets.json: the structure digests of the reference's shipped deploy files as this parser loads them."""
+    import json
+    from mscnn_b200.net import Net
+    from oracle.build_ref import REF
+    from test_net_cpu import SHIPPED_DEPLOY, net_structure
+    out = {p: net_structure(Net(str(REF / "examples" / p / "mscnn_deploy.prototxt"))) for p, _ in SHIPPED_DEPLOY}
+    (OUT / "shipped_deploy_nets.json").write_text(json.dumps(out, indent=1) + "\n")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "full":
         main_full(tuple(sys.argv[2:]) or ("8s", "wider", "7s2x"))
@@ -230,6 +312,12 @@ if __name__ == "__main__":
         main_wider()
     elif len(sys.argv) > 1 and sys.argv[1] == "8s":
         main_8s()
+    elif len(sys.argv) > 1 and sys.argv[1] == "port":
+        main_port()
+    elif len(sys.argv) > 1 and sys.argv[1] == "isolated":
+        main_isolated()
+    elif len(sys.argv) > 1 and sys.argv[1] == "deploy":
+        main_deploy()
     else:
         main()
         main_8s()

@@ -48,6 +48,19 @@ def make_dataset(root: Path, n_images: int = 24, seed: int = 7, with_alpha: bool
     return ids, {k: np.asarray(v, dtype=np.float64).reshape(-1, 6) for k, v in dets.items()}
 
 
+def write_oriented_car_results(res: Path, ids, rows) -> None:
+    """KITTI result files under res/data carrying a valid alpha per Car row (switches the orientation statistics on);
+    no Pedestrian / Cyclist rows."""
+    rng = np.random.default_rng(0)
+    (res / "data").mkdir(parents=True)
+    for pos, img in enumerate(ids, start=1):
+        lines = []
+        for x in rows["Car"][rows["Car"][:, 0] == pos]:
+            lines.append(f"Car -1 -1 {rng.uniform(-3, 3):.2f} {x[1]:.2f} {x[2]:.2f} {x[1] + x[3]:.2f} {x[2] + x[4]:.2f} "
+                         f"-1 -1 -1 -1000 -1000 -1000 -10 {x[5] * 1000:.2f} \n")
+        (res / "data" / f"{img:06d}.txt").write_text("".join(lines))
+
+
 def rows_to_padded(rows: np.ndarray, n_images: int):
     """[img x y w h score] rows -> (dets [N][max][5] float32, counts [N]) as Net.detect returns them."""
     counts = np.array([(rows[:, 0] == i + 1).sum() for i in range(n_images)], dtype=np.int32)

@@ -1,23 +1,20 @@
 """KITTI result writer / evaluator glue (SURVEY.md 8(f)-4), host-only C-ABI entries mscnn_kitti_*.
 
 Oracle: the reference's own tool examples/kitti_result/eval/evaluate_object.cpp compiled VERBATIM
-(oracle/build_ref.py -> oracle/_ref/evaluate_object).  Where it is present the statistics files of both are
-compared byte for byte on seeded synthetic label sets; the same comparison against files the reference tool
-wrote here is committed under tests/golden/kitti_eval/ (tests/golden/make_kitti_golden.py) for boxes without
-the reference.  The two MATLAB writer steps (dlmwrite / writeLabels record formats) are restated from the
-scripts and are parity-unpinned beyond the format checks below."""
-import shutil
-import subprocess
+(oracle/build_ref.py -> oracle/_ref/evaluate_object).  The statistics files it wrote for seeded synthetic label sets
+are committed under tests/golden/kitti_eval/ (tests/golden/make_kitti_golden.py), and the files of this evaluator are
+compared with them byte for byte.  The two MATLAB writer steps (dlmwrite / writeLabels record formats) are restated
+from the scripts and are parity-unpinned beyond the format checks below."""
 from pathlib import Path
 
 import numpy as np
 import pytest
 
-from kitti_synth import make_dataset, rows_to_padded
+from kitti_synth import make_dataset, rows_to_padded, write_oriented_car_results
 
 ROOT = Path(__file__).resolve().parent.parent
-REF_TOOL = ROOT / "oracle" / "_ref" / "evaluate_object"
 GOLDEN = Path(__file__).resolve().parent / "golden" / "kitti_eval"
+GOLDEN_CASES = {(7, 24): ".", (11, 40): "seed11_n40", (3, 5): "seed3_n5"}
 
 
 def _write_results(root, rows, n_images, comp="res"):
@@ -50,51 +47,47 @@ def test_det_file_and_label_formats(tmp_path):
     assert len(b) == 2 and b[1].startswith("Car -1 -1 -10 5.00 6.00 12.00 14.00 ")
 
 
+def _statistics(res):
+    """{path under the result directory: bytes} of every statistics / plot-data file an evaluation wrote."""
+    return {str(f.relative_to(res)): f.read_bytes() for f in [*res.glob("stats_*.txt"), *res.glob("plot/*.txt")]}
+
+
+def _golden_statistics(d):
+    return {f.name.replace("plot_", "plot/", 1) if f.name.startswith("plot_") else f.name: f.read_bytes()
+            for f in d.glob("*.txt")}
+
+
 @pytest.mark.parametrize("seed,n", [(7, 24), (11, 40), (3, 5)])
-@pytest.mark.skipif(not REF_TOOL.exists(), reason="oracle/_ref/evaluate_object not built (needs /root/reference)")
 def test_evaluate_byte_identical_to_reference_tool(tmp_path, seed, n):
+    """Every file this evaluator writes equals what the reference tool wrote for the same result files; no
+    orientation statistics without a valid alpha."""
     from mscnn_b200 import kitti
     ids, rows = make_dataset(tmp_path, n_images=n, seed=seed)
     ours = _write_results(tmp_path, rows, n, "ours")
-    theirs = tmp_path / "theirs"
-    shutil.copytree(ours / "data", theirs / "data")
     ap = kitti.evaluate(tmp_path / "label_2", ours, tmp_path / "val.txt")
-    r = subprocess.run([str(REF_TOOL), str(tmp_path / "label_2"), str(theirs), str(tmp_path / "val.txt")],
-                       capture_output=True, text=True, timeout=300)
-    assert "done" in r.stdout, r.stdout + r.stderr
+    got, want = _statistics(ours), _golden_statistics(GOLDEN / GOLDEN_CASES[seed, n])
+    assert sorted(got) == sorted(want)
+    for rel in want:
+        assert got[rel] == want[rel], rel
     for cls in ("car", "pedestrian", "cyclist"):
-        for rel in (f"stats_{cls}_detection.txt", f"plot/{cls}_detection.txt"):
-            assert (ours / rel).read_bytes() == (theirs / rel).read_bytes(), rel
         assert not (ours / f"stats_{cls}_orientation.txt").exists()
-        assert not (theirs / f"stats_{cls}_orientation.txt").exists()
         tab = np.loadtxt(ours / f"plot/{cls}_detection.txt")
         assert np.allclose(ap[cls], 100 * tab[0:41:4, 1:4].mean(0), atol=1e-4)
 
 
-@pytest.mark.skipif(not REF_TOOL.exists(), reason="oracle/_ref/evaluate_object not built (needs /root/reference)")
 def test_evaluate_with_orientation_and_missing_classes(tmp_path):
     """Result files that carry a valid alpha switch the orientation statistics on; classes never detected are
     not evaluated (evaluate_object.cpp:124-134)."""
     from mscnn_b200 import kitti
     ids, rows = make_dataset(tmp_path, n_images=16, seed=21)
-    rng = np.random.default_rng(0)
-    for comp in ("ours", "theirs"):
-        (tmp_path / comp / "data").mkdir(parents=True)
-    for pos, img in enumerate(ids, start=1):
-        lines = []
-        for x in rows["Car"][rows["Car"][:, 0] == pos]:
-            lines.append(f"Car -1 -1 {rng.uniform(-3, 3):.2f} {x[1]:.2f} {x[2]:.2f} {x[1] + x[3]:.2f} {x[2] + x[4]:.2f} "
-                         f"-1 -1 -1 -1000 -1000 -1000 -10 {x[5] * 1000:.2f} \n")
-        for comp in ("ours", "theirs"):
-            (tmp_path / comp / "data" / f"{img:06d}.txt").write_text("".join(lines))
+    write_oriented_car_results(tmp_path / "ours", ids, rows)
     ap = kitti.evaluate(tmp_path / "label_2", tmp_path / "ours", tmp_path / "val.txt")
-    subprocess.run([str(REF_TOOL), str(tmp_path / "label_2"), str(tmp_path / "theirs"), str(tmp_path / "val.txt")],
-                   capture_output=True, text=True, timeout=300, check=True)
+    got, want = _statistics(tmp_path / "ours"), _golden_statistics(GOLDEN / "orientation_seed21_n16")
+    assert sorted(got) == sorted(want)
     for rel in ("stats_car_detection.txt", "stats_car_orientation.txt", "plot/car_detection.txt", "plot/car_orientation.txt"):
-        assert (tmp_path / "ours" / rel).read_bytes() == (tmp_path / "theirs" / rel).read_bytes(), rel
+        assert got[rel] == want[rel], rel
     assert ap["pedestrian"] is None and ap["cyclist"] is None and ap["car"] is not None
     assert not (tmp_path / "ours" / "stats_pedestrian_detection.txt").exists()
-    assert not (tmp_path / "theirs" / "stats_pedestrian_detection.txt").exists()
 
 
 def test_evaluate_against_committed_reference_output(tmp_path):

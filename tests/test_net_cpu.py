@@ -1,6 +1,8 @@
 """Host-side logic of the drop-in boundary, runnable without a GPU: the text-format reader, the
 Caffe-API mirror's Net construction (split insertion, blob names and shapes, output order,
 parameter shapes), the generated model zoo, and the exported C ABI."""
+import hashlib
+import json
 import re
 import subprocess
 from pathlib import Path
@@ -8,8 +10,11 @@ from pathlib import Path
 import numpy as np
 import pytest
 
+from oracle.build_ref import REF, present
+
 ROOT = Path(__file__).resolve().parent.parent
-REF_EX = Path("/root/reference/examples")
+REF_EX = REF / "examples"
+GOLD = Path(__file__).resolve().parent / "golden"
 
 
 def test_capi_exports_every_declared_symbol():
@@ -121,29 +126,38 @@ def test_unknown_field_is_rejected():
             'layer { bottom: "d" top: "p" name: "p" type: "Pooling" pooling_param { kernel_size: 2 bogus_field: 3 } }\n')
 
 
-@pytest.mark.skipif(not REF_EX.exists(), reason="reference tree not mounted")
-@pytest.mark.parametrize("ref_path,gen", [
+SHIPPED_DEPLOY = [
     ("kitti_car/mscnn-8s-768-trainval", ("kitti", (768, 2560, 8, False))),
     ("kitti_car/mscnn-7s-576", ("kitti", (576, 1920, 7, False))),
     ("kitti_car/mscnn-7s-576-2x", ("kitti", (576, 1920, 7, True))),
     ("widerface/mscnn-12s-2x", ("widerface", (512, 512))),
     ("kitti_car/cascade-mscnn-7s-576-2x", ("kitti_cascade", (576, 1920))),
     ("widerface/cascade-mscnn-12s-align", ("widerface_cascade", (512, 512))),
-])
+]
+
+
+def net_structure(net):
+    """sha256 of the canonical JSON of each thing a loaded net exposes: wiring, parameter and blob shapes, the settings
+    of every layer."""
+    parts = {"layer_names": net.layer_names, "layer_types": net.layer_types, "blob_names": net.blob_names,
+             "layers": net.layers(), "blob_shapes": [net.blob_shape(b) for b in net.blob_names],
+             "layer_param_strings": net.layer_param_strings()}
+    return {k: hashlib.sha256(json.dumps(v).encode()).hexdigest() for k, v in parts.items()}
+
+
+@pytest.mark.parametrize("ref_path,gen", SHIPPED_DEPLOY)
 def test_shipped_deploy_files_load_unchanged_and_match_generated(ref_path, gen):
+    """The reference's shipped <ref_path>/mscnn_deploy.prototxt, loaded unchanged, is recorded in
+    tests/golden/shipped_deploy_nets.json (tests/golden/make_golden.py deploy); the generated net must equal it."""
     from mscnn_b200 import models
     from mscnn_b200.net import Net
-    shipped = Net(str(REF_EX / ref_path / "mscnn_deploy.prototxt"))
-    generated = Net(getattr(models, gen[0])(*gen[1]))
-    assert shipped.layer_names == generated.layer_names
-    assert shipped.layer_types == generated.layer_types
-    assert shipped.blob_names == generated.blob_names
-    assert shipped.layers() == generated.layers()
-    assert [shipped.blob_shape(b) for b in shipped.blob_names] == [generated.blob_shape(b) for b in generated.blob_names]
-    assert shipped.layer_param_strings() == generated.layer_param_strings()
+    shipped = json.loads((GOLD / "shipped_deploy_nets.json").read_text())[ref_path]
+    generated = net_structure(Net(getattr(models, gen[0])(*gen[1])))
+    for part, digest in shipped.items():
+        assert generated[part] == digest, part
 
 
-@pytest.mark.skipif(not REF_EX.exists(), reason="reference tree not mounted")
+@pytest.mark.skipif(not present(REF_EX), reason="the reference tree is not readable here")
 def test_every_shipped_deploy_net_loads():
     """All 23 mscnn_deploy.prototxt files of the reference's model zoo (KITTI car / ped-cyc, Caltech,
     CityPersons, WIDER FACE, plain and cascade) parse, wire up and shape-infer unchanged."""

@@ -201,35 +201,50 @@ def test_e2e_kitti_7s_2x_vs_reference(cuda):
     assert _match_rows(got_ps, ref_ps, 1e-3) >= 0.97
 
 
+def _synthetic_map(shape, scale):
+    """Seeded stand-in for a trunk feature map (a ReLU output) that the stage-isolated tests feed to this net; the
+    reference build was fed the same map (tests/golden/make_golden.py isolated)."""
+    rng = np.random.default_rng(1709)
+    return (np.maximum(rng.standard_normal(shape), 0) * scale).astype(np.float32)
+
+
+def _isolated_protos():
+    """kind -> (deploy text, input n/h/w, feature map the stages read, first stage layer)."""
+    from mscnn_b200 import models
+    return {"head_7s": (models.kitti(96, 320, 7, False, batch=1), (1, 96, 320), "conv4_3", "roi_pool_org"),
+            "cascade_kitti": (models.kitti_cascade(96, 320, batch=2), (2, 96, 320), "conv4_3_2x", "roi_pool_org"),
+            "cascade_wider": (models.widerface_cascade(128, 192, batch=2), (2, 128, 192), "conv4_3", "roi_grid_org")}
+
+
+def _run_isolated(kind):
+    """This net's stages after the feature map, fed with the reference's proposals and the seeded map."""
+    proto, (n, h, w), feat, first = _isolated_protos()[kind]
+    g = np.load(GOLD / f"isolated_{kind}.npz")
+    net = _build(proto, n, h, w)
+    net.forward_only()                                   # our own trunk and proposals, then replaced
+    fmap = _synthetic_map(tuple(net.blob_shape(feat)), float(g["fmap_scale"][0]))
+    for b in net.blob_names:      # every Split top of the feature map / the proposals that the stages read
+        if b.startswith(feat + "_") and "_split_" in b:
+            net.set_input(b, fmap)
+        if b.startswith("proposals_proposals_0_split_"):
+            net.set_input(b, g["proposals"])
+    net.forward_only(start=first)
+    return net, g
+
+
 def test_head_stage_isolated_vs_reference(cuda):
     """ROIPooling x2 + Concat + roi_c1 + fc6 + cls/bbox fed with the REFERENCE's proposals (no
     discrete decision upstream differs): every output row must be within 1e-3."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not present")
-    from mscnn_b200 import models, synth
-    proto = models.kitti(96, 320, 7, False, batch=1)
-    rnet = ref.RefNet(proto, is_path=False)
-    layers = [(n, t, rnet.param_shapes(n)) for n, t in zip(rnet.layer_names, rnet.layer_types)]
-    w = synth.make_weights(layers)
-    rnet.set_params(w)
-    img = synth.make_images(1, 96, 320)
-    rnet.set_blob("data", img)
-    rnet.forward()
-    net = _build(proto, 1, 96, 320)
-    net.forward_only()                                   # our own trunk
-    props = rnet.blob("proposals")
-    conv4_3 = rnet.blob("conv4_3")
-    # inject the reference's conv4_3 and proposals into the blobs the head reads
-    for k in (2, 3):
-        net.set_input(f"conv4_3_relu4_3_0_split_{k}", conv4_3)
-    for k in (0, 1):
-        net.set_input(f"proposals_proposals_0_split_{k}", props)
-    net.forward_only(start="roi_pool_org")
+    net, g = _run_isolated("head_7s")
     for name in ("roi_c1", "fc6", "cls_pred", "bbox_pred"):
-        a, r = net.blob(name), rnet.blob(name)
-        assert a.shape == r.shape, name
-        m2 = float(np.mean(r.astype(np.float64) ** 2))
+        a = net.blob(name)
+        if name + "__sub" in g:
+            assert a.shape == tuple(g[name + "__shape"]), name
+            a, r, m2 = a.reshape(-1)[::997], g[name + "__sub"], float(g[name + "__m2"][0])
+        else:
+            r = g[name]
+            assert a.shape == r.shape, name
+            m2 = float(np.mean(r.astype(np.float64) ** 2))
         err = np.abs(a - r) / (np.abs(r) + np.sqrt(m2))
         assert err.max() <= 1e-3, (name, float(err.max()))
 
@@ -331,38 +346,17 @@ def test_e2e_cascade_vs_reference(cuda, kind):
 
 @pytest.mark.parametrize("kind", ["kitti", "wider"])
 def test_cascade_stages_isolated_vs_reference(cuda, kind):
-    """The three detection stages fed with the REFERENCE's feature map and proposals (run live through
-    oracle/_ref): no discrete decision upstream differs, so rows line up one to one."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not present")
-    from mscnn_b200 import models, synth
-    if kind == "kitti":
-        proto, (n, h, w), feat, first = models.kitti_cascade(96, 320, batch=2), (2, 96, 320), "conv4_3_2x", "roi_pool_org"
-    else:
-        proto, (n, h, w), feat, first = models.widerface_cascade(128, 192, batch=2), (2, 128, 192), "conv4_3", "roi_grid_org"
-    rnet = ref.RefNet(proto, is_path=False)
-    layers = [(nm, t, rnet.param_shapes(nm)) for nm, t in zip(rnet.layer_names, rnet.layer_types)]
-    rnet.set_params(synth.make_weights(layers))
-    rnet.set_blob("data", synth.make_images(n, h, w))
-    rnet.forward()
-    net = _build(proto, n, h, w)
-    net.forward_only()
-    fmap, props = rnet.blob(feat), rnet.blob("proposals")
-    for b in net.blob_names:      # every Split top of the feature map / the proposals that the stages read
-        if b.startswith(feat + "_") and "_split_" in b:
-            net.set_input(b, fmap)
-        if b.startswith("proposals_proposals_0_split_"):
-            net.set_input(b, props)
-    net.forward_only(start=first)
+    """The three detection stages fed with the REFERENCE's proposals and the same feature map as the reference
+    build: no discrete decision upstream differs, so rows line up one to one."""
+    net, g = _run_isolated(f"cascade_{kind}")
     names = ["cls_pred", "bbox_pred", "proposals_2nd", "cls_pred_2nd", "bbox_pred_2nd", "proposals_3rd", "cls_pred_3rd",
              "bbox_pred_3rd", "output_bbox_1st", "output_bbox_2nd", "output_bbox_3rd", "cls_prob_1st", "cls_prob_2nd",
              "cls_prob_3rd"] + (["cls_prob_1st_3rd", "cls_prob_2nd_3rd", "cls_prob_3rd_avg"] if kind == "wider" else [])
     worst = {}
     for name in names:
-        a, r = net.blob(name), rnet.blob(name)
-        assert a.shape == r.shape, name
-        a, r = a.reshape(a.shape[0], -1), r.reshape(r.shape[0], -1)
+        a, r = net.blob(name), g[name]          # the reference's rows g["rows"]
+        assert a.shape == tuple(g[name + "__shape"]), name
+        a, r = a[g["rows"]].reshape(len(r), -1), r.reshape(len(r), -1)
         if name.startswith(("proposals", "output_bbox")):     # boxes: relative to the box extent
             ext = np.maximum(np.maximum(r[:, 3] - r[:, 1], r[:, 4] - r[:, 2]), 1.0)[:, None]
             err = np.abs(a - r) / ext

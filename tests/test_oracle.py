@@ -8,16 +8,16 @@
  (b) golden vectors generated from oracle/_ref = the reference's own layer code compiled verbatim
      (tests/golden/make_golden.py): BoxOutput and ROIPooling(pad_ratio), for which the reference
      ships no test at all;
- (c) when oracle/_ref is present (it is wherever /root/reference was mounted at build time):
-     direct port-vs-reference comparison on random inputs, bit-exact for the integer/ordering
-     parts.
+ (c) port vs the reference build on seeded random inputs, bit-exact for the integer/ordering
+     parts: the reference's outputs for those inputs are in tests/golden/port_vs_reference.npz
+     (tests/golden/make_golden.py port).
 """
 from pathlib import Path
 
 import numpy as np
 import pytest
 
-from oracle import port, ref
+from oracle import port
 
 GOLD = Path(__file__).resolve().parent / "golden"
 
@@ -216,11 +216,9 @@ def test_cascade_detect_postprocess_basics():
 
 
 # ------------------------------------------------------ (c) port vs the verbatim reference build
-needs_ref = pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built (needs /root/reference)")
-
-
-@needs_ref
-def test_port_box_output_vs_reference_random():
+def _box_output_case():
+    """(deploy text, params by layer, input blobs, output blobs) of one reference run; make_golden.py port stores
+    the reference's output blobs for it."""
     rng = np.random.default_rng(11)
     shapes = [(12, 40), (12, 40), (6, 20), (6, 20), (3, 10)]
     fields, rates = [60, 84, 120, 168, 240], [8, 8, 16, 16, 32]
@@ -229,22 +227,16 @@ def test_port_box_output_vs_reference_random():
     proto += "layer { " + " ".join(f'bottom: "m{j}"' for j in range(5)) + ' top: "r" top: "rs" name: "p" type: "BoxOutput" '
     proto += 'box_output_param { fg_thr: -2 iou_thr: 0.65 nms_type: "IOU" ' + " ".join(f"field_w: {f} field_h: {f}" for f in fields)
     proto += " " + " ".join(f"downsample_rate: {r}" for r in rates) + " max_nms_num: 150 } }"
-    net = ref.RefNet(proto, is_path=False)
-    maps = []
+    blobs = {}
     for j, (h, w) in enumerate(shapes):
         m = rng.standard_normal((2, 9, h, w)).astype(np.float32)
         m[:, :5] *= 3
         m[:, 5:] *= 0.5
-        maps.append(m)
-        net.set_blob(f"m{j}", m)
-    net.forward()
-    rois, sc, _, _ = port.box_output(maps, fields, fields, rates, fg_thr=-2.0, iou_thr=0.65, max_nms_num=150)
-    assert np.array_equal(rois, net.blob("r").reshape(-1, 5))
-    assert np.array_equal(sc, net.blob("rs").reshape(-1, 6))
+        blobs[f"m{j}"] = m
+    return proto, {}, blobs, ["r", "rs"]
 
 
-@needs_ref
-def test_port_layers_vs_reference_random():
+def _layers_case():
     rng = np.random.default_rng(12)
     proto = '''input: "x" input_dim: 2 input_dim: 16 input_dim: 9 input_dim: 11
 layer { name: "c" type: "Convolution" bottom: "x" top: "c" convolution_param { num_output: 8 kernel_size: 5 pad: 2 } }
@@ -253,28 +245,15 @@ layer { name: "p" type: "Pooling" bottom: "c" top: "p" pooling_param { pool: MAX
 layer { name: "a" type: "Pooling" bottom: "c" top: "a" pooling_param { pool: AVE kernel_size: 2 stride: 2 } }
 layer { name: "d" type: "Deconvolution" bottom: "c" top: "d" convolution_param { kernel_size: 4 stride: 2 num_output: 8 group: 8 pad: 1 weight_filler: { type: "bilinear" } bias_term: false } }
 layer { name: "f" type: "InnerProduct" bottom: "p" top: "f" inner_product_param { num_output: 7 } }'''
-    net = ref.RefNet(proto, is_path=False)
     x = rng.standard_normal((2, 16, 9, 11)).astype(np.float32)
     w = rng.standard_normal((8, 16, 5, 5)).astype(np.float32) * 0.1
     b = rng.standard_normal(8).astype(np.float32)
     wf = rng.standard_normal((7, 8 * 5 * 6)).astype(np.float32) * 0.1
     bf = rng.standard_normal(7).astype(np.float32)
-    net.set_param("c", 0, w); net.set_param("c", 1, b); net.set_param("f", 0, wf); net.set_param("f", 1, bf)
-    net.set_blob("x", x)
-    net.forward()
-    c = port.relu(port.conv2d(x, w, b, pad=2))
-    np.testing.assert_allclose(c, net.blob("c"), rtol=1e-5, atol=1e-5)
-    c = net.blob("c")
-    assert np.array_equal(port.pool(c, 2, 2), net.blob("p"))
-    np.testing.assert_allclose(port.pool(c, 2, 2, mode="AVE"), net.blob("a"), rtol=1e-6)
-    from mscnn_b200 import synth
-    np.testing.assert_allclose(port.deconv_depthwise(c, np.broadcast_to(synth.bilinear_kernel(4), (8, 1, 4, 4)).copy()),
-                               net.blob("d"), rtol=1e-6, atol=1e-7)
-    np.testing.assert_allclose(port.inner_product(net.blob("p"), wf, bf), net.blob("f"), rtol=1e-5, atol=1e-5)
+    return proto, {"c": [w, b], "f": [wf, bf]}, {"x": x}, ["c", "p", "a", "d", "f"]
 
 
-@needs_ref
-def test_port_cascade_layers_vs_reference_random():
+def _cascade_layers_case():
     rng = np.random.default_rng(21)
     n, c, h, w, r = 2, 16, 14, 22, 60
     proto = f'''input: "x" input_dim: {n} input_dim: {c} input_dim: {h} input_dim: {w}
@@ -285,16 +264,54 @@ layer {{ bottom: "x" bottom: "r" top: "a" name: "a" type: "ROIAlign" roi_pooling
 layer {{ bottom: "b" bottom: "r" top: "d" name: "d" type: "DecodeBBox" bbox_reg_param {{ bbox_mean: 0.1 bbox_mean: -0.1 bbox_mean: 0.05 bbox_mean: 0 bbox_std: 0.1 bbox_std: 0.1 bbox_std: 0.2 bbox_std: 0.2 }} }}
 layer {{ bottom: "s" top: "sm" name: "sm" type: "Softmax" softmax_param {{ axis: 1 }} }}
 layer {{ bottom: "s" top: "sl" name: "sl" type: "Softmax" softmax_param {{ axis: -1 }} }}'''
-    net = ref.RefNet(proto, is_path=False)
     x = rng.standard_normal((n, c, h, w)).astype(np.float32)
     x1 = rng.uniform(-10, 80, r); y1 = rng.uniform(-10, 50, r)
     rois = np.stack([rng.integers(0, n, r), x1, y1, x1 + rng.uniform(-5, 60, r), y1 + rng.uniform(-5, 40, r)], 1).astype(np.float32)
     b = rng.standard_normal((r, 8)).astype(np.float32)
     s = (rng.standard_normal((r, 5, 3, 2)) * 3).astype(np.float32)
-    net.set_blob("x", x); net.set_blob("r", rois.reshape(r, 5, 1, 1)); net.set_blob("b", b.reshape(r, 8, 1, 1))
-    net.set_blob("s", s)
-    net.forward()
-    assert np.array_equal(port.roi_align(x, rois, 4, 7, 0.25, 0.125), net.blob("a"))
-    assert np.array_equal(port.decode_bbox(b, rois, (0.1, -0.1, 0.05, 0), (0.1, 0.1, 0.2, 0.2)), net.blob("d").reshape(r, 5))
-    np.testing.assert_allclose(port.softmax(s, 1), net.blob("sm"), rtol=2e-6, atol=1e-10)
-    np.testing.assert_allclose(port.softmax(s, 3), net.blob("sl"), rtol=2e-6, atol=1e-10)
+    return proto, {}, {"x": x, "r": rois.reshape(r, 5, 1, 1), "b": b.reshape(r, 8, 1, 1), "s": s}, ["a", "d", "sm", "sl"]
+
+
+PORT_CASES = {"box_output": _box_output_case, "layers": _layers_case, "cascade_layers": _cascade_layers_case}
+
+
+def _reference(case):
+    """The reference build's output blobs for PORT_CASES[case]."""
+    g = np.load(GOLD / "port_vs_reference.npz")
+    return {k.split("__", 1)[1]: g[k] for k in g.files if k.startswith(case + "__")}
+
+
+def test_port_box_output_vs_reference_random():
+    _, _, maps, _ = _box_output_case()
+    ref = _reference("box_output")
+    rois, sc, _, _ = port.box_output(list(maps.values()), [60, 84, 120, 168, 240], [60, 84, 120, 168, 240],
+                                     [8, 8, 16, 16, 32], fg_thr=-2.0, iou_thr=0.65, max_nms_num=150)
+    assert np.array_equal(rois, ref["r"].reshape(-1, 5))
+    assert np.array_equal(sc, ref["rs"].reshape(-1, 6))
+
+
+def test_port_layers_vs_reference_random():
+    _, params, blobs, _ = _layers_case()
+    (w, b), (wf, bf), x = params["c"], params["f"], blobs["x"]
+    ref = _reference("layers")
+    c = port.relu(port.conv2d(x, w, b, pad=2))
+    np.testing.assert_allclose(c, ref["c"], rtol=1e-5, atol=1e-5)
+    c = ref["c"]
+    assert np.array_equal(port.pool(c, 2, 2), ref["p"])
+    np.testing.assert_allclose(port.pool(c, 2, 2, mode="AVE"), ref["a"], rtol=1e-6)
+    from mscnn_b200 import synth
+    np.testing.assert_allclose(port.deconv_depthwise(c, np.broadcast_to(synth.bilinear_kernel(4), (8, 1, 4, 4)).copy()),
+                               ref["d"], rtol=1e-6, atol=1e-7)
+    np.testing.assert_allclose(port.inner_product(ref["p"], wf, bf), ref["f"], rtol=1e-5, atol=1e-5)
+
+
+def test_port_cascade_layers_vs_reference_random():
+    _, _, blobs, _ = _cascade_layers_case()
+    x, s = blobs["x"], blobs["s"]
+    r = len(blobs["r"])
+    rois, b = blobs["r"].reshape(r, 5), blobs["b"].reshape(r, 8)
+    ref = _reference("cascade_layers")
+    assert np.array_equal(port.roi_align(x, rois, 4, 7, 0.25, 0.125)[::6], ref["a"])      # every 6th ROI stored
+    assert np.array_equal(port.decode_bbox(b, rois, (0.1, -0.1, 0.05, 0), (0.1, 0.1, 0.2, 0.2)), ref["d"].reshape(r, 5))
+    np.testing.assert_allclose(port.softmax(s, 1), ref["sm"], rtol=2e-6, atol=1e-10)
+    np.testing.assert_allclose(port.softmax(s, 3), ref["sl"], rtol=2e-6, atol=1e-10)
